@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repository's CUDA path
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle/_ref + restatement)
     python bench.py --workload single30k|kitti120k|micro1m   # the other BASELINE configs (side lines, same JSON shape)
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed (.npy)
 
 Default workload `batch8x30k`: a step = one pass of the hot path (4 grid subsamplings + 13 radius searches + 10 KPConv +
 23 unary convs + BN/LeakyReLU/pools) over one batch of 8 stacked synthetic 3DMatch-shaped fragments of 30 000 points
@@ -15,6 +16,7 @@ workload it prints -- full-size fragments; when K + W full steps would not finis
 timed steps and says so (`steps_run`), it never shrinks the fragments.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -30,6 +32,7 @@ if ROOT not in sys.path:
 
 WORKLOADS = ("batch8x30k", "single30k", "kitti120k", "micro1m")
 REF_ARM_BUDGET_S = 200.0          # the reference arm cuts STEPS (never points) to stay inside this
+DUMP_BUDGET_BYTES = 64 << 20      # --dump-outputs writes at most this much
 
 
 def parse():
@@ -42,7 +45,32 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true", help="one batch at a time on one stream")
     ap.add_argument("--no-graph", action="store_true", help="do not replay the step as a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the arrays the last timed step returned as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(d, arrays):
+    """Write {name: array} as d/<name>.npy in float32 (float64 for integers that float32 cannot hold exactly). The
+    inputs are seeded, so two builds given the same arguments can be compared file by file. An array larger than its
+    even share of DUMP_BUDGET_BYTES is cut to a fixed, seeded sample of rows, whose indices go to <name>_rows.npy."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BUDGET_BYTES // max(len(arrays), 1)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype.kind in "iu":
+            a = a.astype(np.float32 if a.size == 0 or np.abs(a).max() < (1 << 24) else np.float64)
+        elif a.dtype != np.float64:
+            a = a.astype(np.float32)
+        if a.nbytes > share:
+            row_bytes = a.nbytes // a.shape[0] + 8
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], share // row_bytes, replace=False))
+            np.save(os.path.join(d, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a))
 
 
 def peaks():
@@ -148,7 +176,7 @@ def cpu_reference_run(cfg, params, clouds, limits, steps, warmup, budget_s):
     with ThreadPoolExecutor(T) as ex:
         for it in range(warmup + steps):
             t0 = time.perf_counter()
-            list(ex.map(lambda p: cpu_one_fragment(cfg, params, p, limits, use_ref), clouds))
+            last = list(ex.map(lambda p: cpu_one_fragment(cfg, params, p, limits, use_ref), clouds))
             dt = time.perf_counter() - t0
             if it >= warmup:
                 times.append(dt)
@@ -165,7 +193,8 @@ def cpu_reference_run(cfg, params, clouds, limits, steps, warmup, budget_s):
               "(TensorFlow not installable)") % (
         len(clouds), n_pts, T, str(blas), nproc, len(times), warmup,
         "reference C++ cores (oracle/_ref)" if use_ref else "C restatement (oracle/liboracle.so)")
-    return times, dict(kind=kind, cores=nproc, threads=T, sample=sample, points_per_step=n_pts)
+    return times, dict(kind=kind, cores=nproc, threads=T, sample=sample, points_per_step=n_pts,
+                       outputs=dict(features=np.concatenate(last, 0)))
 
 
 def cpu_micro_run(P, steps, warmup):
@@ -180,13 +209,14 @@ def cpu_micro_run(P, steps, warmup):
     for it in range(warmup + steps):
         t0 = time.perf_counter()
         sp, sb = sub(P, n, 0.03)
-        nbf(sp, sp, sb, sb, 0.075)
+        nb = nbf(sp, sp, sb, sb, 0.075)
         if it >= warmup:
             times.append(time.perf_counter() - t0)
     return times, dict(kind="reference" if use_ref else "port", cores=os.cpu_count() or 1, threads=1,
                        sample="1 000 000 raw points per step: grid subsampling dl 0.03 then radius neighbours r 0.075 of "
                               "the subsampled cloud, single host thread (one TF op), %d timed steps after %d warm-up "
-                              "(median)" % (len(times), warmup), points_per_step=int(P.shape[0]))
+                              "(median)" % (len(times), warmup), points_per_step=int(P.shape[0]),
+                       outputs=dict(subsampled_points=sp, subsampled_lengths=sb, neighbors=nb))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -207,6 +237,8 @@ class ClockSampler:
                                       stdout=self.f, stderr=subprocess.DEVNULL)
         except OSError:
             pass
+        else:      # a benchmark that raises before stop() must not leave the sampler polling
+            atexit.register(self.p.kill)
 
     def stop(self):
         out = dict(sm_mhz=None, sm_max_mhz=None, reasons=[])
@@ -286,6 +318,8 @@ def main():
                                       sample=info["sample"]),
                     e2e=dict(value=value, unit="points/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0),
                     gpu_launches=0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, info["outputs"])
         print(json.dumps(line))
         return
 
@@ -315,12 +349,24 @@ def main():
 
     gather_cap = max(64, n_points // 128)    # rows reserved per rank for the coarsest-level descriptors (~1.5x actual)
 
+    # (result, device level counts or None) of the most recent step: what --dump-outputs writes
+    last_out = [None]
+
     def step_resident():
         out = enc(P_dev, L_dev, bbox=bbox, decoder=False)
         desc = out["F"][-1]
+        last_out[0] = (desc, None)
         if world > 1:      # the one exchange step: NCCL all-gather of the per-fragment descriptors (sync-free)
             desc, _ = all_gather_descriptors_padded(desc, out["inputs"]["lengths"][-1], gather_cap)
         return desc
+
+    def host_outputs():
+        """This rank's coarsest-level encoder features of the most recent step, rows beyond the level count dropped
+        (the graph pipeline returns a capacity-sized buffer)."""
+        res, counts = last_out[0]
+        if counts is not None:
+            res = res[:int(counts[len(LIMITS) - 1].item())]
+        return dict(features=res.cpu().numpy())
 
     def step_e2e():
         # the call a user makes: host buffers in, descriptors out (host) -- H2D and D2H inside the timed region
@@ -439,6 +485,7 @@ def main():
                         host_counts.copy_(last_counts[0], non_blocking=True)
                 if mark is not None:
                     mark.record(pipe.s_enc)
+            last_out[0] = (res, last_counts[0])
             return res
 
         prime(src_p, src_l, src_bbox)
@@ -468,8 +515,9 @@ def main():
         barrier()
         wall = (time.perf_counter() - t0) * 1000.0 / steps      # synchronised on both sides
         # consecutive encoders alternate between w streams and finish in bursts: a step's time is the completion
-        # interval averaged over a window of w steps (w = 1: plain consecutive intervals)
-        w = len(getattr(pipe, "s_encs", [None]))
+        # interval averaged over a window of w steps (w = 1: plain consecutive intervals; fewer steps than streams:
+        # the whole region)
+        w = min(len(getattr(pipe, "s_encs", [None])), steps)
         per_step = [marks[i].elapsed_time(marks[i + w]) / w for i in range(steps - w + 1)]
         launches = (_lib.launch_count() - n0) // max(steps, 1)
         if hasattr(pipe, "check"):
@@ -488,10 +536,12 @@ def main():
     if args.no_pipeline:
         st, launches = timed(step_resident, args.steps, 1)
         clocks = sampler.stop() if sampler else None
+        outputs = host_outputs() if args.dump_outputs else None
         st_e2e, _ = timed(step_e2e, args.steps, 1)
     else:
         st, launches = timed_pipelined(args.steps, max(args.warmup, 3), False)
         clocks = sampler.stop() if sampler else None
+        outputs = host_outputs() if args.dump_outputs else None
         st_e2e, _ = timed_pipelined(args.steps, max(args.warmup, 3), True)
     # headline = the MEDIAN step (max over ranks); mean and max are reported beside it: a single host stall moves the
     # mean of 20 steps by tens of percent and says nothing about the path
@@ -613,6 +663,8 @@ def main():
                             "sizes stay on the device, no host synchronisation (encoder.GraphPipeline)")))
         line["single_batch_latency_ms"] = seq["median"]
         line["single_batch_latency_ms_max"] = seq["max"]
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -636,6 +688,8 @@ def main_micro(args, world, rank, local_rank):
         times, info = cpu_micro_run(P, min(args.steps, 5), min(args.warmup, 1))
         st = stats_ms([t * 1000.0 for t in times])
         value = info["points_per_step"] / (st["median"] / 1000.0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, info["outputs"])
         print(json.dumps(dict(base, impl="reference", value=value, ms_per_step=st["median"], steps_run=len(times),
                               cpu_baseline=dict(value=value, unit="points/s", cores=info["cores"], kind=info["kind"],
                                                 sample=info["sample"]),
@@ -665,6 +719,8 @@ def main_micro(args, world, rank, local_rank):
         sp, sb = sub(p)
         nb = nbr(sp, sb)
         res["M"], res["cols"] = int(sp.shape[0]), int(nb.shape[1])
+        if args.dump_outputs:
+            res["out"] = (sp, sb, nb)
         return sp, sb, nb
 
     def timed(fn, steps, warmup):
@@ -684,6 +740,9 @@ def main_micro(args, world, rank, local_rank):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     st, launches = timed(lambda: step(P_dev), args.steps, max(args.warmup, 3))
     clocks = sampler.stop() if sampler else None
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = dict(zip(("subsampled_points", "subsampled_lengths", "neighbors"), (t.cpu().numpy() for t in res["out"])))
 
     def e2e():
         sp, sb, nb = step(P_pin.to(dev, non_blocking=True))
@@ -713,6 +772,8 @@ def main_micro(args, world, rank, local_rank):
         cpu = dict(value=info["points_per_step"] / (cst["median"] / 1000.0), unit="points/s", cores=info["cores"],
                    kind=info["kind"], sample=info["sample"], ms_per_step=cst["median"])
     if rank == 0:
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         n = P.shape[0] * world
         print(json.dumps(dict(base, value=n / (st["median"] * 1e-3), ms_per_step=st["median"],
                               ms_per_step_mean=st["mean"], ms_per_step_max=st["max"],

@@ -9,6 +9,7 @@ Two back-ends, both CPU:
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s CPU-baseline legs may import this module.
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -277,3 +278,22 @@ def sort_rows(a):
         return a, np.zeros((0,), np.int64)
     order = np.lexsort(tuple(a[:, k] for k in range(a.shape[1] - 1, -1, -1)))
     return a[order], order
+
+
+def digest(a):
+    """[shape, sha256 of the C-ordered bytes]: the stored form of a reference output too large to keep as an array
+    (tests/golden/reference_digests.json)."""
+    a = np.ascontiguousarray(a)
+    return [list(a.shape), hashlib.sha256(a.tobytes()).hexdigest()]
+
+
+def pyramid_digests(pyr):
+    """Digests of an input pyramid (kpconv_np.descriptor_input_pyramid form): per level the barycenter bits, the
+    stack lengths and the int32 neighbour / pool / upsample matrices."""
+    out = []
+    for l in range(len(pyr["points"])):
+        d = dict(points=digest(_f32(pyr["points"][l]).view(np.uint32)), lengths=_i32(pyr["lengths"][l]).tolist())
+        for key in ("neighbors", "pools", "upsamples"):
+            d[key] = digest(_i32(pyr[key][l]))
+        out.append(d)
+    return out

@@ -1,10 +1,10 @@
 """Formats either side of the hot path (SURVEY.md §8 f3/f4): TF checkpoint bundles, parameters.txt, PLY, and the
 per-fragment output arrays. CPU only.
 
-Known answers from the reference's own artefacts (read only where /root/reference exists, i.e. in the build
-container): the 10 kernel-point tensors inside results_kitti/Log_11011605/snapshots/snap-61 must equal the
-kernel_points/epoch61/*.ply files the trainer wrote from the same variables, bit for bit, and the variable names
-of all three released snapshots must be exactly the names the host mirror looks up.
+Known answers from the reference's own artefacts (tests/golden/released/, files of the released models copied verbatim
+by scripts/make_golden_reference.py): the 10 kernel-point tensors inside results_kitti/Log_11011605/snapshots/snap-61
+must equal the kernel_points/epoch61/*.ply files the trainer wrote from the same variables, bit for bit, and the
+variable names of all three released snapshots must be exactly the names the host mirror looks up.
 """
 import glob
 import os
@@ -15,8 +15,31 @@ import pytest
 from d3feat_b200 import io_utils, synth
 from d3feat_b200 import tf_checkpoint as ck
 
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present on this machine")
+REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "released")
+
+
+def released_snapshot(tmp_path, log, snap, payload=None):
+    """Prefix of a tensor bundle made of the released snapshot's real .index and a data shard of the real length in
+    which only the tensors of `payload` ({name: raw bytes}) hold their real bytes (the rest is left as a hole)."""
+    prefix = str(tmp_path / ("snap-%d" % snap))
+    with open(os.path.join(REF, log, "snapshots", "snap-%d.index" % snap), "rb") as fh:
+        index = fh.read()
+    with open(prefix + ".index", "wb") as fh:
+        fh.write(index)
+    _, entries = ck.read_index(prefix)
+    with open(prefix + ".data-00000-of-00001", "wb") as fh:
+        fh.truncate(max(e["offset"] + e["size"] for e in entries.values()))
+        for name, raw in (payload or {}).items():
+            fh.seek(entries[name]["offset"])
+            fh.write(raw.tobytes())
+    return prefix
+
+
+def model_variables(prefix):
+    """{name: (shape, dtype)} of the variables load_params returns, from the bundle's index alone."""
+    _, entries = ck.read_index(prefix)
+    return {n[len(ck.MODEL_SCOPE):]: (tuple(e["shape"]), np.dtype(ck._DTYPES[e["dtype"]])) for n, e in entries.items()
+            if n.startswith(ck.MODEL_SCOPE) and not n.endswith(ck._OPTIMIZER_SLOTS)}
 
 
 def test_crc32c_known_answers():
@@ -66,12 +89,15 @@ def test_bundle_corruption_is_detected(tmp_path):
         ck.read_index(prefix)
 
 
-@needs_ref
-def test_released_snapshots_known_answers():
+def test_released_snapshots_known_answers(tmp_path):
     log = os.path.join(REF, "results_kitti", "Log_11011605")
-    params = ck.load_params(os.path.join(log, "snapshots", "snap-61"))
+    z = np.load(os.path.join(REF, "snap-61_kernel_points.npz"))
+    prefix = released_snapshot(tmp_path, "results_kitti/Log_11011605", 61,
+                               {k.replace("|", "/"): z[k] for k in z.files})
+    names = [k.replace("|", "/") for k in z.files]
+    params = {n[len(ck.MODEL_SCOPE):]: a for n, a in ck.read_checkpoint(prefix, names=names).items()}   # CRC-checked
     plys = sorted(glob.glob(os.path.join(log, "kernel_points", "epoch61", "*.ply")))
-    assert len(plys) == 10
+    assert len(plys) == 10 and len(params) == 10
     for f in plys:
         base = os.path.basename(f)[:-4]                                      # layer_1_resnetb_0_conv2
         names = [n for n in params if n.endswith("kernel_points") and n.replace("/", "_").startswith(base + "_k")]
@@ -81,20 +107,20 @@ def test_released_snapshots_known_answers():
     # variable names / shapes == what the host mirror asks for, for every released model
     for log, snap in (("results_kitti/Log_11011605", 61), ("results/Log_contraloss", 54), ("results/Log_circleloss", 48)):
         cfg = io_utils.load_config(os.path.join(REF, log))
-        got = ck.load_params(os.path.join(REF, log, "snapshots", "snap-%d" % snap))
+        got = model_variables(released_snapshot(tmp_path, log, snap))
         want = synth.make_params(cfg, 0)
         assert set(got) == set(want), log
-        assert all(got[k].shape == tuple(np.shape(want[k])) and got[k].dtype == np.float32 for k in got), log
+        assert all(got[k] == (tuple(np.shape(want[k])), np.float32) for k in got), log
         assert cfg.num_layers == 5 and cfg.first_features_dim == 64 and cfg.num_kernel_points == 15
 
 
-@needs_ref
 def test_config_and_ply_readers_on_reference_files():
     cfg = io_utils.load_config(os.path.join(REF, "results", "Log_contraloss"))
     assert cfg.architecture[0] == "simple" and cfg.architecture[-1] == "last_unary" and len(cfg.architecture) == 19
     assert abs(cfg.first_subsampling_dl - 0.03) < 1e-9 and cfg.KP_influence == "linear" and cfg.modulated is False
-    pts = io_utils.read_ply_points(os.path.join(REF, "demo_data", "cloud_bin_0.ply"))
-    assert pts.shape == (258342, 3) and pts.dtype == np.float32 and np.isfinite(pts).all()
+    # demo_data/cloud_bin_0.ply (CloudCompare header, 258342 vertices) cut to its first 2048 vertices
+    pts = io_utils.read_ply_points(os.path.join(REF, "demo_data", "cloud_bin_0_head.ply"))
+    assert pts.shape == (2048, 3) and pts.dtype == np.float32 and np.isfinite(pts).all()
 
 
 def test_ply_ascii_and_big_endian(tmp_path):
@@ -130,40 +156,3 @@ def test_keypoint_selection_and_writers(tmp_path):
     assert (np.diff(s[:, 0]) >= 0).all()                    # ascending: evaluate.py takes the LAST 250 rows
     assert np.array_equal(k[-1], pts[np.argmax(sc)]) and np.array_equal(d[-1], desc[np.argmax(sc)])
 
-
-@needs_ref
-def test_released_model_registers_the_demo_pair_through_the_restatement():
-    """Behavioural known answer for the TF-graph restatement (oracle/kpconv_np.py): with the RELEASED 3DMatch weights,
-    BN statistics and kernel points (read by tf_checkpoint.py) the numpy encoder + decoder + detector must produce
-    descriptors that register the reference's demo fragments (demo_registration.py flow); with the weights shuffled
-    inside each tensor the matches must collapse. scripts/oracle_released_demo.py is the full-size version
-    (2500 keypoints: 53 % inlier ratio, overlap 6 % -> 81 %, tests/golden/released_demo_summary.json)."""
-    import importlib.util
-    from scipy.spatial import cKDTree
-    from oracle import native as on
-    spec = importlib.util.spec_from_file_location(
-        "oracle_released_demo", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "scripts",
-                                             "oracle_released_demo.py"))
-    demo = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(demo)
-    if not on.have_ref():
-        on.build(ref=True)
-    cfg = io_utils.load_config(os.path.join(REF, "results", "Log_contraloss"))
-    params = ck.load_params(os.path.join(REF, "results", "Log_contraloss", "snapshots", "snap-54"))
-    clouds = []
-    for i in (0, 1):
-        raw = io_utils.read_ply_points(os.path.join(REF, "demo_data", "cloud_bin_%d.ply" % i))
-        clouds.append(on.ref_batch_subsampling(raw, np.array([raw.shape[0]], np.int32), cfg.first_subsampling_dl)[0])
-    limits = [37, 35, 36, 38, 38]                       # demo.calibrate(cfg, clouds), tests/golden/released_demo_summary.json
-    d, s = zip(*(demo.describe(cfg, params, limits, c) for c in clouds))
-    assert all(np.allclose(np.linalg.norm(x, axis=1), 1.0, atol=1e-4) for x in d)
-    kp = [np.argsort(x[:, 0])[-1500:] for x in s]
-    d0, d1 = d[0][kp[0]], d[1][kp[1]]
-    nn01 = cKDTree(d1).query(d0)[1]
-    mutual = np.nonzero(cKDTree(d0).query(d1)[1][nn01] == np.arange(d0.shape[0]))[0]
-    src, dst = clouds[0][kp[0]][mutual], clouds[1][kp[1]][nn01[mutual]]
-    r, t, inl = demo.ransac(src, dst, iters=3000)
-    assert mutual.size > 100 and inl.sum() / mutual.size > 0.3
-    before = np.mean(cKDTree(clouds[1]).query(clouds[0])[0] < 0.05)
-    after = np.mean(cKDTree(clouds[1]).query(clouds[0] @ r.T + t)[0] < 0.05)
-    assert before < 0.15 and after > 0.6
