@@ -56,6 +56,16 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// A operand from tensor memory (M = 128: TMEM lane = row of A, column = one tf32 k-element; K = 8 columns per MMA)
+__device__ __forceinline__ void umma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc,
+                                             uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
@@ -75,6 +85,20 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
   for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
+}
+
+// a warp writes 32 columns of its 32 TMEM lanes (lane l -> TMEM lane (taddr >> 16) + l), then waits for the store
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const float (&v)[32]) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
+      ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]), "f"(v[8]),
+        "f"(v[9]), "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]), "f"(v[16]), "f"(v[17]),
+        "f"(v[18]), "f"(v[19]), "f"(v[20]), "f"(v[21]), "f"(v[22]), "f"(v[23]), "f"(v[24]), "f"(v[25]), "f"(v[26]),
+        "f"(v[27]), "f"(v[28]), "f"(v[29]), "f"(v[30]), "f"(v[31])
+      : "memory");
+  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 }
 
 // explicit shared-window accesses: the aligned stage pointer is derived through integer arithmetic, so plain C++

@@ -4,12 +4,16 @@
 //
 //   C[M,N] = epilogue( rowscale[m] * (A[M,K] @ W[K,N]) )
 //
-// * A is the activation matrix (row-major fp32 in global memory). It is loaded by 4 producer warps with coalesced
-//   128-bit loads, split into (hi, lo) in registers and written to shared memory in the canonical K-major
-//   SWIZZLE_128B layout the UMMA descriptor expects (rows of 128 B = 32 fp32, 16-byte chunks XOR-ed with row%8).
-// * W is static: it is packed once (pack_weight_kernel) into K-major [Npad, Kpad] hi/lo images.
-// * One elected thread of warp 4 issues the MMAs (M = 128, N = BN, K = 8 per instruction); a 3-stage
-//   mbarrier ring overlaps the producers with the tensor pipe; tcgen05.commit releases stages / signals the epilogue.
+// * A is the activation matrix (row-major fp32 in global memory). Producer warp w copies the raw rows it owns,
+//   [32w, 32w+32), into a swizzled shared-memory slot (cp.async, 128-bit, coalesced); lane l reads its own row back,
+//   splits it into (hi, lo) in registers and writes both to tensor memory (tcgen05.st): TMEM lane = row, one
+//   column per k-element. The MMAs take A from TMEM, so shared memory carries only the raw copy of A and the B
+//   images. (D3F_TC_A_SMEM=1 keeps the round-2 path for A/B timing: both A images in shared memory, in the K-major
+//   SWIZZLE_128B layout of the UMMA descriptor.)
+// * W is static: it is packed once (pack_weight_kernel) into K-major [Npad, Kpad] hi/lo images, fetched by TMA.
+// * One elected thread of warp 4 issues the MMAs (M = 128, N = BN, K = 8 per instruction, three per K step); a
+//   1-4 stage mbarrier ring overlaps the producers with the tensor pipe; tcgen05.commit releases stages / signals the
+//   epilogue.
 // * Epilogue: warps 0-3 read their 32 TMEM lanes (tcgen05.ld 32x32b), apply rowscale / BN / bias / residual /
 //   LeakyReLU and store rows straight to global memory.
 #include <stdlib.h>
@@ -65,27 +69,45 @@ int tc_pack_weight(const float* W, int K, int N, float* packed, cudaStream_t str
 // ~ -1.1e-8 * K relative for all-positive data (scripts/tc_accuracy_probe.py). The k-chunks are therefore
 // rotated over kAcc independent TMEM accumulators (2 x 128 or 4 x 64 / 4 x 32 columns) that the epilogue adds
 // in registers with round-to-nearest: the truncation chain per accumulator is kAcc times shorter.
-// ACC = 0: the default rotation (2 x 128 or 4 x 64 / 4 x 32 columns: <= 256 TMEM columns per CTA, two CTAs fit in
-// the 512 columns). ACC = 1: a single accumulator for GEMMs of <= 4 k-chunks (K <= 128: bias < 1.5e-6), so that
-// four or five small CTAs share an SM.
-template <int BN, int ACC>
+// ACC = 0: the default rotation (2 x 128, 4 x 64 / 4 x 32 columns; 2 x 64 for the two-CTA <64,2> ring with the A
+// operand in TMEM, where 4 x 64 + 128 A columns would not leave room for a second CTA -- K of that variant stays
+// <= 1024 in the encoder: bias < 5.6e-6). ACC = 1: a single accumulator for GEMMs of <= 4 k-chunks (K <= 128: bias
+// < 1.5e-6), so that four small CTAs share an SM.
+// A_SMEM = false (default): the split A operand lives in TMEM, 64 columns per ring stage ([hi 32 | lo 32]) after
+// the accumulators. A_SMEM = true: both A images in shared memory (the round-2 operand path, kept for A/B timing).
+// TMEM allocation (a power of two >= 32) / ring stages / shared memory / CTAs per SM, A in TMEM vs A in smem:
+//   <32,1,1>   32 + 64 -> 128 | 1 |  25 KB | 4        (A_SMEM:  32 | 1 |  41 KB | 4)
+//   <64,1,1>   64 + 64 -> 128 | 1 |  33 KB | 4        (A_SMEM:  64 | 1 |  49 KB | 4)
+//   <32,2,0>  128 + 128 -> 256 | 2 |  49 KB | 2       (A_SMEM: 128 | 2 |  81 KB | 2)
+//   <64,2,0>  128 + 128 -> 256 | 2 |  65 KB | 2       (A_SMEM: 256 | 2 |  97 KB | 2)
+//   <128,2,0> 256 + 128 -> 512 | 2 |  97 KB | 1       (A_SMEM: 256 | 2 | 129 KB | 1)
+//   <32,4,0>  128 + 256 -> 512 | 4 |  97 KB | 1       (A_SMEM: 128 | 4 | 161 KB | 1)
+//   <64,4,0>  256 + 256 -> 512 | 4 | 129 KB | 1       (A_SMEM: 256 | 4 | 193 KB | 1)
+//   <128,3,0> 256 + 192 -> 512 | 3 | 145 KB | 1       (A_SMEM: 256 | 3 | 193 KB | 1)
+// (CTAs per SM: the launch bounds' register budget; shared memory and TMEM admit at least as many.)
+template <int BN, int STAGES, int ACC, bool A_SMEM>
 struct TcAcc {
-  static constexpr int kAcc = ACC > 0 ? ACC : (BN >= 128 ? 2 : 4);
-  static constexpr int kCols = kAcc * BN;   // power of two, 32 <= kCols <= 512
+  static constexpr int kAcc = ACC > 0 ? ACC : (BN >= 128 ? 2 : ((BN == 64 && STAGES == 2 && !A_SMEM) ? 2 : 4));
+  static constexpr int kACol = kAcc * BN;                    // first TMEM column of the A ring
+  static constexpr int kUsed = kACol + (A_SMEM ? 0 : 64 * STAGES);
+  static constexpr int kCols = kUsed <= 32 ? 32 : kUsed <= 64 ? 64 : kUsed <= 128 ? 128 : kUsed <= 256 ? 256 : 512;
+  static_assert(kUsed <= 512, "TMEM plan exceeds 512 columns");
 };
 
 // ring depth = prefetch distance + 1. Skinny-K GEMMs (<= 4 k-chunks) take 2 stages so that two CTAs share an SM and
 // overlap each other's load / MMA / epilogue phases; long-K GEMMs take the deepest ring that fits (one CTA per SM).
-template <int BN, int STAGES>
+// A stage holds the raw (A in TMEM) or the hi and lo (A_SMEM) images of the A tile, then the B hi and lo images.
+template <int BN, int STAGES, bool A_SMEM>
 struct TcSmem {
   static constexpr int kStages = STAGES;
-  static constexpr int kABytes = kTcBM * 128;  // one image (hi or lo) of the A tile
+  static constexpr int kABytes = kTcBM * 128;  // one image of the A tile
   static constexpr int kBBytes = BN * 128;
-  static constexpr int kStageBytes = 2 * kABytes + 2 * kBBytes;
+  static constexpr int kBOff = (A_SMEM ? 2 : 1) * kABytes;
+  static constexpr int kStageBytes = kBOff + 2 * kBBytes;
   static constexpr int kTotal = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/;
 };
 
-template <int BN, int STAGES, int ACC>
+template <int BN, int STAGES, int ACC, bool A_SMEM>
 __global__ void __launch_bounds__(kTcThreads, STAGES == 1 ? 4 : ((STAGES == 2 && BN <= 64) ? 2 : 1))
 tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1, const float* __restrict__ Bp,
                float* __restrict__ C, int Mcap, int N, int K, int Kpad, int Npad, int chunks_per_split, Epilogue ep) {
@@ -93,7 +115,8 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
   const int M = ep.m_dev ? min(Mcap, max(__ldg(ep.m_dev) - ep.m_off, 0)) : Mcap;
   if ((int)blockIdx.y * kTcBM >= M) return;   // CTA-uniform, before any barrier / TMEM allocation
   extern __shared__ uint8_t smem_raw[];
-  using S = TcSmem<BN, STAGES>;
+  using S = TcSmem<BN, STAGES, A_SMEM>;
+  using P = TcAcc<BN, STAGES, ACC, A_SMEM>;
   constexpr int kStages = S::kStages;
   // 1024 B alignment: SWIZZLE_128B atoms are 8 rows x 128 B and the swizzle uses absolute address bits
   uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
@@ -118,7 +141,7 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
   }
   if (warp == 4) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)TcAcc<BN, ACC>::kCols)
+                 "r"((uint32_t)P::kCols)
                  : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
@@ -128,18 +151,24 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp < 4) {
-    // ===================== producers: global --cp.async--> swizzled stage --(in-place hi/lo split)--> UMMA =====
-    // Every thread owns fixed 16-byte pieces of the stage (row = it*16 + rsub, chunk = tid & 7). It copies them
-    // asynchronously kStages-1 k-chunks ahead (A raw fp32 into the "hi" image, pre-split B into both images; rows
-    // beyond M / K are zero-filled), and when ITS OWN copy group of chunk kt has landed (cp.async.wait_group is
-    // per thread, so no extra barrier) it splits its A pieces in place: hi overwrites the raw value, lo goes to the
-    // second image. No register staging: the number of loads in flight is bounded by the stage ring only.
-    const int chunk = tid & 7;      // 16-byte chunk inside the 128-byte row
-    const int rsub = tid >> 3;      // 0..15: row inside a 16-row slab
+    // ===================== producers: global --cp.async--> swizzled raw stage --hi/lo split--> operand =========
+    // The raw fp32 A tile is copied asynchronously kStages-1 k-chunks ahead (rows beyond M / K zero-filled), the
+    // pre-split B images by TMA. When a thread's copy group of chunk kt has landed (cp.async.wait_group is per
+    // thread) the A values are split into (hi, lo):
+    //   A in TMEM: warp w copies the 32 rows it owns, [32w, 32w+32) (eight lanes per 128-byte row segment); after
+    //     wait_group + __syncwarp lane l reads its own row 32w + l back (eight 16-byte chunks; the swizzle puts the
+    //     rows of a quarter-warp in distinct bank groups) and writes hi / lo to TMEM lane 32w + l, columns
+    //     [kACol + 64 s, +32) / [kACol + 64 s + 32, +32). Warp w may only touch TMEM lanes [32w, 32w+32).
+    //   A_SMEM: every thread owns fixed 16-byte pieces of the stage and splits them in place (hi overwrites the raw
+    //     value, lo goes to the second image), in the K-major SWIZZLE_128B layout the UMMA descriptor reads.
+    const int chunk = A_SMEM ? (tid & 7) : (lane & 7);      // 16-byte chunk inside the 128-byte row
+    constexpr int kRowStep = A_SMEM ? 16 : 4;                 // rows one copy instruction covers
+    const int rbase = A_SMEM ? (tid >> 3) : warp * 32 + (lane >> 3);
     auto issue_chunk = [&](int kt) {
       const int s = kt % kStages;
       const uint32_t ph = (uint32_t)(kt / kStages) & 1u;
       mbar_wait(smem_u32(&bars[kStages + s]), ph ^ 1u);      // stage free (its MMAs retired)
+      if constexpr (!A_SMEM) tc_fence_after();               // the TMEM A stage is rewritten after this wait
       uint8_t* st = smem + s * S::kStageBytes;
       // the A operand is [A | A2] along K when A2 is given (K1 = columns of A, a multiple of the k-chunk): a whole
       // k-chunk comes from one of the two row-major matrices
@@ -155,8 +184,8 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
         }
       }
 #pragma unroll
-      for (int it = 0; it < kTcBM / 16; ++it) {
-        const int row = it * 16 + rsub;
+      for (int it = 0; it < (A_SMEM ? kTcBM : 32) / kRowStep; ++it) {
+        const int row = rbase + it * kRowStep;
         const int gm = m0 + row;
         const uint32_t off = (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
         const bool ok = gm < M && k0 < ld;
@@ -168,8 +197,8 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
         const uint32_t full = smem_u32(&bars[s]);
         const float* slab = Bp + (size_t)(kt0 + kt) * 2 * Npad * 32 + (size_t)n0 * 32;
         mbar_arrive_expect_tx(full, 2u * S::kBBytes);
-        tma_bulk_g2s(smem_u32(st + 2 * S::kABytes), slab, S::kBBytes, full);
-        tma_bulk_g2s(smem_u32(st + 2 * S::kABytes + S::kBBytes), slab + (size_t)Npad * 32, S::kBBytes, full);
+        tma_bulk_g2s(smem_u32(st + S::kBOff), slab, S::kBBytes, full);
+        tma_bulk_g2s(smem_u32(st + S::kBOff + S::kBBytes), slab + (size_t)Npad * 32, S::kBBytes, full);
       }
     };
     for (int i = 0; i < kStages - 1; ++i) {
@@ -188,29 +217,47 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
       } else {
         asm volatile("cp.async.wait_group %0;" ::"n"(kStages >= 2 ? kStages - 2 : 0) : "memory");   // chunk kt landed
       }
-      // all of this thread's pieces are read before anything is written back: the loads are independent of the
-      // in-place stores (which the compiler could not prove), so the eight shared-memory round trips overlap
-      float4 x[kTcBM / 16];
       const uint32_t st_s = smem_u32(st);
+      if constexpr (A_SMEM) {
+        // all of this thread's pieces are read before anything is written back: the loads are independent of the
+        // in-place stores (which the compiler could not prove), so the eight shared-memory round trips overlap
+        float4 x[kTcBM / 16];
 #pragma unroll
-      for (int it = 0; it < kTcBM / 16; ++it) {
-        const int row = it * 16 + rsub;
-        const uint32_t off = (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
-        x[it] = lds128(st_s + off);
-      }
+        for (int it = 0; it < kTcBM / 16; ++it) {
+          const int row = it * 16 + rbase;
+          const uint32_t off = (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
+          x[it] = lds128(st_s + off);
+        }
 #pragma unroll
-      for (int it = 0; it < kTcBM / 16; ++it) {
-        const int row = it * 16 + rsub;
-        const uint32_t off = (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
-        float4 hi, lo;
-        split_tf32(x[it].x, hi.x, lo.x);
-        split_tf32(x[it].y, hi.y, lo.y);
-        split_tf32(x[it].z, hi.z, lo.z);
-        split_tf32(x[it].w, hi.w, lo.w);
-        sts128(st_s + off, hi);
-        sts128(st_s + S::kABytes + off, lo);
+        for (int it = 0; it < kTcBM / 16; ++it) {
+          const int row = it * 16 + rbase;
+          const uint32_t off = (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
+          float4 hi, lo;
+          split_tf32(x[it].x, hi.x, lo.x);
+          split_tf32(x[it].y, hi.y, lo.y);
+          split_tf32(x[it].z, hi.z, lo.z);
+          split_tf32(x[it].w, hi.w, lo.w);
+          sts128(st_s + off, hi);
+          sts128(st_s + S::kABytes + off, lo);
+        }
+        fence_proxy_async();   // generic-proxy writes -> visible to the tensor core (async proxy)
+      } else {
+        __syncwarp();          // the other lanes' pieces of this warp's rows have landed too
+        const int row = warp * 32 + lane;
+        float hi[32], lo[32];
+#pragma unroll
+        for (int c = 0; c < 8; ++c) {
+          const float4 x = lds128(st_s + (uint32_t)row * 128u + (uint32_t)((c ^ (row & 7)) << 4));
+          split_tf32(x.x, hi[4 * c + 0], lo[4 * c + 0]);
+          split_tf32(x.y, hi[4 * c + 1], lo[4 * c + 1]);
+          split_tf32(x.z, hi[4 * c + 2], lo[4 * c + 2]);
+          split_tf32(x.w, hi[4 * c + 3], lo[4 * c + 3]);
+        }
+        const uint32_t ta = tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)(P::kACol + 64 * s);
+        tmem_st32(ta, hi);
+        tmem_st32(ta + 32u, lo);
+        tc_fence_before();     // the completed TMEM stores -> ordered before the MMA issuer's wait on full[s]
       }
-      fence_proxy_async();   // generic-proxy writes -> visible to the tensor core (async proxy)
       mbar_arrive(smem_u32(&bars[s]));
       if constexpr (kStages > 1) {
         // refill the stage that MMA(kt-1) is about to release, kStages-1 chunks ahead
@@ -229,7 +276,7 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
     const int row = warp * 32 + lane;      // TMEM lane == tile row; warp w may only touch lanes [32w, 32w+32)
     const int gm = m0 + row;
     const float rs = (ep.rowscale != nullptr && gm < M) ? ep.rowscale[gm] : 1.f;
-    const int nacc = nk < TcAcc<BN, ACC>::kAcc ? nk : TcAcc<BN, ACC>::kAcc;
+    const int nacc = nk < P::kAcc ? nk : P::kAcc;
     const uint32_t tile = smem_u32(smem) + (uint32_t)warp * (32 * 33 * 4);
     const int rows_here = min(32, M - (m0 + warp * 32));   // rows of this warp that exist (<= 0: none)
     const bool has_bn = ep.bn_scale != nullptr, has_bias = ep.bias != nullptr, has_res = ep.residual != nullptr;
@@ -309,15 +356,24 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
       tc_fence_after();
       if (lane == 0) {
         const uint32_t sa = smem_u32(smem + s * S::kStageBytes);
-        const uint64_t a_hi = make_smem_desc(sa), a_lo = make_smem_desc(sa + S::kABytes);
-        const uint64_t b_hi = make_smem_desc(sa + 2 * S::kABytes), b_lo = make_smem_desc(sa + 2 * S::kABytes + S::kBBytes);
+        const uint64_t b_hi = make_smem_desc(sa + S::kBOff), b_lo = make_smem_desc(sa + S::kBOff + S::kBBytes);
+        const uint32_t d = tmem_base + (uint32_t)((kt % P::kAcc) * BN);
 #pragma unroll
         for (int j = 0; j < kTcBK / 8; ++j) {
           const uint64_t adv = (uint64_t)((j * 32) >> 4);   // +32 B per K = 8 step inside the swizzle atom
-          const uint32_t d = tmem_base + (uint32_t)((kt % TcAcc<BN, ACC>::kAcc) * BN);
-          umma_tf32(d, a_hi + adv, b_hi + adv, idesc, (kt >= TcAcc<BN, ACC>::kAcc || j != 0) ? 1u : 0u);
-          umma_tf32(d, a_lo + adv, b_hi + adv, idesc, 1u);
-          umma_tf32(d, a_hi + adv, b_lo + adv, idesc, 1u);
+          const uint32_t acc = (kt >= P::kAcc || j != 0) ? 1u : 0u;
+          if constexpr (A_SMEM) {
+            const uint64_t a_hi = make_smem_desc(sa), a_lo = make_smem_desc(sa + S::kABytes);
+            umma_tf32(d, a_hi + adv, b_hi + adv, idesc, acc);
+            umma_tf32(d, a_lo + adv, b_hi + adv, idesc, 1u);
+            umma_tf32(d, a_hi + adv, b_lo + adv, idesc, 1u);
+          } else {
+            // A stage s: hi at columns [kACol + 64 s, +32), lo at [+32, +64); K = 8 columns per MMA
+            const uint32_t a_hi = tmem_base + (uint32_t)(P::kACol + 64 * s + 8 * j);
+            umma_tf32_ts(d, a_hi, b_hi + adv, idesc, acc);
+            umma_tf32_ts(d, a_hi + 32u, b_hi + adv, idesc, 1u);
+            umma_tf32_ts(d, a_hi, b_lo + adv, idesc, 1u);
+          }
         }
         umma_commit(smem_u32(&bars[kStages + s]));                 // stage free once these MMAs retire
         if (kt == nk - 1) umma_commit(smem_u32(&bars[2 * kStages]));  // accumulator complete
@@ -330,7 +386,7 @@ tc_gemm_kernel(const float* __restrict__ A, const float* __restrict__ A2, int K1
   if (warp == 4) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base),
-                 "r"((uint32_t)TcAcc<BN, ACC>::kCols)
+                 "r"((uint32_t)P::kCols)
                  : "memory");
   }
 }
@@ -355,20 +411,20 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restr
   }
 }
 
-template <int BN, int STAGES, int ACC = 0>
+template <int BN, bool A_SMEM, int STAGES, int ACC = 0>
 static int launch_tc_s(const float* A, const float* A2, int K1, const float* Bp, float* C, int M, int N, int K,
                        const Epilogue& ep, cudaStream_t stream, int splits, float* split_ws) {
-  using S = TcSmem<BN, STAGES>;
+  using S = TcSmem<BN, STAGES, A_SMEM>;
   static bool configured = false;   // idempotent attribute set; benign if two host threads race
   if (!configured) {
-    D3F_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<BN, STAGES, ACC>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
+    D3F_CUDA(cudaFuncSetAttribute(tc_gemm_kernel<BN, STAGES, ACC, A_SMEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::kTotal));
     configured = true;
   }
   int Kpad = tc_padded_k(K), Npad = tc_padded_n(N);
   const int nk = Kpad / kTcBK;
   if (splits <= 1) {
     dim3 grid(Npad / BN, ceil_div(M, kTcBM), 1);
-    tc_gemm_kernel<BN, STAGES, ACC><<<grid, kTcThreads, S::kTotal, stream>>>(A, A2, K1, Bp, C, M, N, K, Kpad, Npad, nk, ep);
+    tc_gemm_kernel<BN, STAGES, ACC, A_SMEM><<<grid, kTcThreads, S::kTotal, stream>>>(A, A2, K1, Bp, C, M, N, K, Kpad, Npad, nk, ep);
     D3F_LAUNCH_CHECK("tc_gemm_kernel");
     return D3F_OK;
   }
@@ -378,7 +434,7 @@ static int launch_tc_s(const float* A, const float* A2, int K1, const float* Bp,
   raw.rowscale = nullptr; raw.bn_scale = nullptr; raw.bn_shift = nullptr; raw.bias = nullptr; raw.residual = nullptr;
   raw.leaky_alpha = -1.f; raw.row_map = nullptr; raw.m_dev = ep.m_dev; raw.m_off = ep.m_off;
   dim3 grid(Npad / BN, ceil_div(M, kTcBM), splits);
-  tc_gemm_kernel<BN, STAGES, ACC><<<grid, kTcThreads, S::kTotal, stream>>>(A, A2, K1, Bp, split_ws, M, N, K, Kpad, Npad, cps, raw);
+  tc_gemm_kernel<BN, STAGES, ACC, A_SMEM><<<grid, kTcThreads, S::kTotal, stream>>>(A, A2, K1, Bp, split_ws, M, N, K, Kpad, Npad, cps, raw);
   D3F_LAUNCH_CHECK("tc_gemm_kernel");
   long long total = (long long)M * N;
   int blocks = (int)min((total + 255) / 256, (long long)kNumSMs * 8);
@@ -676,7 +732,7 @@ static bool force_deep_ring() {
 }
 static const int kSkinnyChunks = [] { int c = env_int("D3F_TC_SKINNY_CHUNKS", 4); return c < 1 ? 1 : (c > 4 ? 4 : c); }();
 
-template <int BN>
+template <int BN, bool A_SMEM>
 static int launch_tc(const float* A, const float* A2, int K1, const float* Bp, float* C, int M, int N, int K,
                      const Epilogue& ep, cudaStream_t stream, int splits = 1, float* split_ws = nullptr) {
   const int nk_per_cta = ceil_div(tc_padded_k(K) / kTcBK, splits > 1 ? splits : 1);
@@ -687,10 +743,10 @@ static int launch_tc(const float* A, const float* A2, int K1, const float* Bp, f
   // accumulator CTAs, four per SM -- their load / MMA / epilogue phases overlap across CTAs
   if constexpr (BN <= 64) {
     if (nk_per_cta <= kSkinnyChunks && splits <= 1 && ctas > 4ll * kNumSMs && !force_deep_ring())
-      return launch_tc_s<BN, 1, 1>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+      return launch_tc_s<BN, A_SMEM, 1, 1>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
   }
-  if (nk_per_cta <= 4 || (BN <= 64 && ctas > kNumSMs)) return launch_tc_s<BN, 2>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
-  return launch_tc_s<BN, (BN >= 128 ? 3 : 4)>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+  if (nk_per_cta <= 4 || (BN <= 64 && ctas > kNumSMs)) return launch_tc_s<BN, A_SMEM, 2>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+  return launch_tc_s<BN, A_SMEM, (BN >= 128 ? 3 : 4)>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
 }
 
 bool tc_gemm_supported(const float* A, int K) {
@@ -755,10 +811,18 @@ int tc_gemm(const float* A, const float* Bp, float* C, int M, int N, int K, cons
     if (bn == 64) return launch_tc_stream<64>(A, A2, K1, Bp, C, M, N, K, ep, stream);
     return launch_tc_stream<32>(A, A2, K1, Bp, C, M, N, K, ep, stream);
   }
+  // D3F_TC_A_SMEM=1: the A operand through shared memory (both split images), for A/B timing of the two paths
+  if (env_int("D3F_TC_A_SMEM", 0) != 0) {
+    switch (bn) {
+      case 128: return launch_tc<128, true>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+      case 64: return launch_tc<64, true>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+      default: return launch_tc<32, true>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+    }
+  }
   switch (bn) {
-    case 128: return launch_tc<128>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
-    case 64: return launch_tc<64>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
-    default: return launch_tc<32>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+    case 128: return launch_tc<128, false>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+    case 64: return launch_tc<64, false>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
+    default: return launch_tc<32, false>(A, A2, K1, Bp, C, M, N, K, ep, stream, splits, split_ws);
   }
 }
 
